@@ -2,7 +2,7 @@
 """bench.py -- BASELINE.json metric: 256x256x3 slices/sec of the PnP-AdaNet hot path on B200, synthetic data,
 random-init weights.
 
-    python bench.py --gpus N --steps K --warmup W [--config C]     (N>1: launched by torchrun, one rank per GPU)
+    python bench.py --gpus N --steps K --warmup W [--config C] [--dump-outputs DIR]     (N>1: launched by torchrun, one rank per GPU)
     python bench.py --impl reference ...       (the CPU restatement of the reference's TF-1.4 path on the host cores --
                                                 TF-1.4 itself cannot run in this image; same config, time-bounded)
 
@@ -29,6 +29,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 # algorithmic conv/FC FLOPs (2*MAC) per unit, SURVEY 8(d) / Appendix A.5
@@ -258,6 +259,39 @@ class Workload:
         self._fwd_graph = None
 
 
+# --dump-outputs: an output larger than this many elements is written as a fixed, seeded sample of them, so that the files of
+# one run stay under 64 MB in all (at most two such arrays per config)
+DUMP_MAX_ELEMS = 6 * 2 ** 20
+DUMP_SEED = 0
+
+
+def _host_sample(t):
+    t = t.detach()
+    if t.numel() > DUMP_MAX_ELEMS:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(t.numel(), DUMP_MAX_ELEMS, replace=False))
+        t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+    return t.float().cpu().numpy()
+
+
+def dump_outputs(w, out, d):
+    """what the last timed step computed, as <d>/<name>.npy: config 1 the logits [B,256,256,5]; the training configs their
+    losses (float64 scalars) and the parameters the step updated (float32, flat arena order)"""
+    c, tr = w.cfg, w.trainer
+    if c == 1:
+        arrays = {"logits": out}
+    elif c == 2:
+        arrays = {"wce_loss": float(out[0]), "dice_loss": float(out[1]), "params": tr.arena.theta}
+    elif c == 3:
+        arrays = {"dis_loss": tr.loss_value(out), "dis_params": tr.d_arena.theta}
+    else:
+        arrays = {"dis_loss": tr.loss_value(out[0]), "gen_loss": tr.loss_value(out[1]),
+                  "dis_params": tr.d_arena.theta, "gen_params": tr.g_arena.theta}
+    os.makedirs(d, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), _host_sample(v) if torch.is_tensor(v) else np.float64(v))
+    print("bench: wrote %s to %s" % (", ".join(n + ".npy" for n in arrays), d), file=sys.stderr)
+
+
 def _dp_check(w, dist):
     """driver-visible data-parallel evidence (N > 1), computed after the timed loop on a fresh D-step:
       * first-step exchange error: the N-rank update (NCCL all-reduce + fused RMSProp) vs the same optimizer kernel applied to
@@ -329,11 +363,12 @@ def run_ours(a):
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """-> (ms for `steps` calls of fn, what the last call returned)"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for i in range(steps):
-            fn(i)
+            last = fn(i)
         e1.record()
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1)
@@ -341,7 +376,7 @@ def run_ours(a):
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         barrier()
-        return float(t.item())
+        return float(t.item()), last
 
     # kernel launches of one step, counted on an eager step (a graph replay issues the same kernels without host calls)
     l0 = _C.launch_count
@@ -352,9 +387,12 @@ def run_ours(a):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms_total = timed(w.step_resident, a.steps)
+    ms_total, last = timed(w.step_resident, a.steps)
     launches = launches_per_step * a.steps
     clocks = sampler.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:      # before anything below steps the model again
+        dump_outputs(w, last, a.dump_outputs)
+    del last
     ms_step = ms_total / a.steps
     cfgobj = bench_config(a.config, B, a.keep_prob, world)
     slices_per_step = cfgobj["slices_per_step"]
@@ -363,7 +401,7 @@ def run_ours(a):
     # end-to-end through the public Trainer API with host inputs + result read-back
     for i in range(min(2, a.warmup)):
         w.step_e2e(i)
-    ms_e2e = timed(w.step_e2e, a.steps) / a.steps
+    ms_e2e = timed(w.step_e2e, a.steps)[0] / a.steps
     e2e = {"value": slices_per_step / (ms_e2e / 1e3), "unit": "slices/s", "h2d_bytes_per_step": w.h2d, "d2h_bytes_per_step": w.d2h,
            "ms_per_step": ms_e2e}
 
@@ -383,8 +421,7 @@ def run_ours(a):
                 tr.d_step_replay(mr, ct, a.keep_prob)
             tr.g_step_replay(w.dev_pool[i % 3][2], a.keep_prob)
         nd20_step(0)
-        reps = max(2, min(a.steps, 3))
-        ms20 = timed(nd20_step, reps) / reps
+        ms20 = timed(nd20_step, a.steps)[0] / a.steps
         nd20 = {"n_D": 20, "slices_per_step": 41 * B, "ms_per_step": ms20, "value": 41 * B / (ms20 / 1e3), "unit": "slices/s",
                 "cuda_graph": bool(ok and a.graph), "conv_tflops_algorithmic": B * (20 * GF_D_STEP_PER_PAIR + GF_G_STEP_PER_SLICE) / ms20}
         if a.graph:        # back to the joint graph for the roofline pass below (eager) -- nothing else replays after this
@@ -639,7 +676,14 @@ def main():
     ap.add_argument("--graph", dest="graph", action="store_true", default=True, help="replay the step as one CUDA graph (default)")
     ap.add_argument("--no-graph", dest="graph", action="store_false")
     ap.add_argument("--profile", action="store_true", help="per-kernel device-time table of two eager steps (torch.profiler) on stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (same arguments, same inputs: runs of two "
+                         "builds compare output for output)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if a.batch is None:
         a.batch = WORKLOADS[a.config][1]
     if a.backend is None:

@@ -29,7 +29,9 @@ def test_library_exports_every_declared_symbol():
     assert set(declared) == bound, (set(declared) ^ bound)
     assert _C.lib.pnp_version() >= 100
     assert _C.lib.pnp_error_string(100002).decode().startswith("pnp: unsupported")
-    assert _C.lib.pnp_tc_available() == 0          # no device in this container
+    # the tcgen05 path reports itself available exactly on a Blackwell (compute capability 10.x) device
+    on_sm100 = torch.cuda.is_available() and torch.cuda.get_device_capability()[0] == 10
+    assert _C.lib.pnp_tc_available() == int(on_sm100)
 
 
 def test_no_cpu_fallback_product_does_not_import_oracle():
@@ -158,7 +160,9 @@ def test_confusion_matrix_metrics_match_oracle():
 
 
 def _dp_worker(rank, world, port, out):
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank))
+    # host ranks over gloo: hide any GPU, which would otherwise have to exist once per LOCAL_RANK
+    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank),
+                      CUDA_VISIBLE_DEVICES="")
     sys.path.insert(0, ROOT)
     import pnp_b200  # noqa: F401
     from pnp_b200 import parallel
@@ -214,17 +218,17 @@ def test_checkpoint_transplant_chain_baseline_to_gan(tmp_path):
     # conv weights of the frozen segmenter come from the baseline, name for name
     for n in base:
         if "/Variable" in n:
-            assert np.array_equal(v[n].numpy(), base[n]), n
+            assert np.array_equal(v[n].cpu().numpy(), base[n]), n
     # BN: old_bn_list[i] -> pred_bn_list[i]  (the reference's two lists are index-aligned)
     scope_of = {}
     for n in v:
         if "/pred_" in n:
             scope_of[n.split("/", 1)[1]] = n
     for old, new in zip(gold["old_bn_list"], gold["pred_bn_list"]):
-        assert np.array_equal(v[scope_of[new]].numpy(), base[old]), (old, new)
+        assert np.array_equal(v[scope_of[new]].cpu().numpy(), base[old]), (old, new)
     # DAM initialised from the MR front: half_zip_mri_vars[i] -> half_zip_ct_vars[i]
     for m, c_ in zip(gold["half_zip_mri_vars"], gold["half_zip_ct_vars"]):
-        assert np.array_equal(v[c_].numpy(), v[m].numpy()), (m, c_)
+        assert np.array_equal(v[c_].cpu().numpy(), v[m].cpu().numpy()), (m, c_)
     # critics untouched
     for n in v:
         if "cls" in n:
@@ -497,7 +501,7 @@ def test_entry_scripts_read_the_reference_list_files(tmp_path):
     tr.val_stats = lambda x, y, step=None, log_dir=None, detail=False: seen["val"].append(x.clone()) or {}
     tr.train(output_path=str(tmp_path / "seg"), training_iters=3, epochs=1, display_step=2)
     imgs = lambda lst: [truth[p] for p in lst]
-    member = lambda x, pool: any(np.array_equal(x.numpy(), im) for im in pool)
+    member = lambda x, pool: any(np.array_equal(x.cpu().numpy(), im) for im in pool)
     assert len(seen["train"]) == 3 and len(seen["val"]) == 2
     assert all(member(b[k], imgs(mr_train)) for b in seen["train"] for k in range(2))
     assert all(member(b[k], imgs(mr_val)) for b in seen["val"] for k in range(2))

@@ -452,7 +452,9 @@ def test_training_schedule_and_step_feeds_match_the_reference(tmp_path):
         return segment
     tr2 = A.Trainer(A.Full_DRN(3, 5, B, cost_kwargs=dict(COST), network_config=dict(CFG)), num_cls=5, batch_size=B,
                     opt_kwargs={"learning_rate": 3e-4}, train_config=dict(sched["train_config"]))
-    saved = (optim.call, _C.call, rt.stream)
+    # scratch.begin_step() drops its record of the used accumulators; with its zero-fill a no-op here, that record is restored
+    # afterwards, or the next real step on a device would accumulate onto stale sums
+    saved = (optim.call, _C.call, rt.stream, rt.scratch.off, rt.scratch.high)
     optim.call = _C.call = lambda *a, **k: None                      # no kernels: only the Python control flow is exercised
     rt.stream = lambda: None
     x = torch.empty(B, 256, 256, 3, device="meta")
@@ -466,7 +468,7 @@ def test_training_schedule_and_step_feeds_match_the_reference(tmp_path):
             tr2.g_step(x, 0.75)
         g_calls = calls
     finally:
-        optim.call, _C.call, rt.stream = saved
+        optim.call, _C.call, rt.stream, rt.scratch.off, rt.scratch.high = saved
     assert d_calls == [{"stream": "mr", "keep_prob": 0.75, "front_bn": d_feeds[0]["mr_front_bn"], "joint_bn": d_feeds[0]["joint_bn"]},
                        {"stream": "ct", "keep_prob": 0.75, "front_bn": d_feeds[0]["ct_front_bn"], "joint_bn": d_feeds[0]["joint_bn"]}]
     assert g_calls == [{"stream": "ct", "keep_prob": 0.75, "front_bn": g_feeds[0]["ct_front_bn"], "joint_bn": g_feeds[0]["joint_bn"]}]
@@ -582,7 +584,7 @@ def test_segmenter_training_schedule_feeds_and_adam_match_the_reference(tmp_path
     tr2 = S.Trainer(S.Full_DRN(3, 5, B, cost_kwargs={"cross_flag": True, "miu_cross": 1.0, "dice_flag": True, "miu_dice": 1.0}),
                     train_list=[], val_list=[], num_cls=5, batch_size=B, opt_kwargs={"learning_rate": 1e-3}, optimizer="adam")
     tr2.net.forward = forward
-    saved = (optim.call, _C.call, rt.stream)
+    saved = (optim.call, _C.call, rt.stream, rt.scratch.off, rt.scratch.high)      # scratch: as in the adversarial probe above
     optim.call = _C.call = lambda *a, **k: None
     rt.stream = lambda: None
     x = torch.empty(B, 256, 256, 3, device="meta")
@@ -591,7 +593,7 @@ def test_segmenter_training_schedule_feeds_and_adam_match_the_reference(tmp_path
             with pytest.raises(_Stop):
                 fn()
     finally:
-        optim.call, _C.call, rt.stream = saved
+        optim.call, _C.call, rt.stream, rt.scratch.off, rt.scratch.high = saved
     assert calls == [{"keep_prob": 0.75, "main_bn": True, "adapt_bn": True},
                      {"keep_prob": 1.0, "main_bn": True, "adapt_bn": True},
                      {"keep_prob": 1.0, "main_bn": False, "adapt_bn": False}]
